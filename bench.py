@@ -2,6 +2,7 @@
 """bench.py -- the driver-facing benchmark (DESIGN.md section 6 "Measurement").
 
   python bench.py --gpus N --steps K --warmup W            # this repo's GPU engine
+  python bench.py ... --dump-outputs DIR                    # also write the replies of the last timed step to DIR
   python bench.py --impl reference --gpus N --steps K ...   # the reference's own CPU server (oracle/_ref)
 
 Metric (BASELINE.json): committed txns/sec on lock_fasst.  Workload at N = 1: the reference's own lock_fasst trace
@@ -9,14 +10,13 @@ shape (lock_fasst/caladan/trace_init.sh: 24,000,000 lock ids, uniform, 5-10 ids 
 0.2) driven closed-loop by 1,048,576 logical clients through the FaSST protocol of lock_fasst/caladan/client.cc
 against a 36,000,000-slot lock table ("REF" in SURVEY.md 8(d)).  One STEP = one batch of 4 client rounds =
 4,194,304 wire requests.  W + K steps of the closed loop are recorded (every reply of the recording is compared with
-the UNMODIFIED reference server binary fed the same stream); the timed region replays the K recorded steps, device
-resident, in cycles -- the server state is restored from a snapshot at the start of every cycle (inside the timed
-region) so that every cycle reproduces the recording bit for bit -- until it is at least one second long.  Every step
-reads a different 37.7 MB trace segment (K segments >> L2).  At N > 1 every rank drives its own 1,048,576 clients and
-the key space grows with N (36 M slots and 24 M ids PER GPU: constant contention), requests travel to the owning GPU
-through the dispatch / engine / combine step over NVLink; the reference's fixed 36 M / 24 M constants at N > 1, TATP
-and SmallBank on the reference's shard placement, HOT, store GET, lock_2pl, log_server and the UDP front-end are
-reported under "extra".
+the UNMODIFIED reference server binary fed the same stream); the timed region replays the K recorded steps once,
+device resident, from the server state the W warm-up steps left, so that it reproduces the recording bit for bit.
+Every step reads a different 37.7 MB trace segment (K segments >> L2).  At N > 1 every rank drives its own 1,048,576
+clients and the key space grows with N (36 M slots and 24 M ids PER GPU: constant contention), requests travel to
+the owning GPU through the dispatch / engine / combine step over NVLink; the reference's fixed 36 M / 24 M constants
+at N > 1, TATP and SmallBank on the reference's shard placement, HOT, store GET, lock_2pl, log_server and the UDP
+front-end are reported under "extra".
 """
 import argparse
 import json
@@ -30,13 +30,14 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 CLIENTS = 1 << 20
 ROUNDS_PER_STEP = 4
 STEP_REQS = CLIENTS * ROUNDS_PER_STEP
-TIMED_SECONDS = float(os.environ.get("DINT_BENCH_SECONDS", "1.0"))      # minimum length of every timed region
+TIMED_SECONDS = float(os.environ.get("DINT_BENCH_SECONDS", "1.0"))      # minimum length of the extras' timed regions
 # algorithmic bytes per request (SURVEY.md 8(d)): wire in + wire out + state at the reference's field granularity
 FASST_BYTES = {4: 22, 5: 26, 6: 22, 7: 22, 8: 30}          # by reply type
 STORE_GET_BYTES = 186
@@ -177,17 +178,23 @@ def fasst_alg_bytes(resps, msg=9):
     return int(sum(FASST_BYTES[t] * int(cnt[t]) for t in FASST_BYTES)), {str(t): int(cnt[t]) for t in FASST_BYTES}
 
 
-def cycles_for(step_ms, k):
-    return max(1, int(np.ceil(TIMED_SECONDS * 1e3 / max(step_ms * k, 1e-6))))
+def dump_replies(out_dir, raw, n_sample=1 << 21):
+    """--dump-outputs: lock_fasst reply records `raw` (wire bytes) as one float64 .npy per wire field (exact for every
+    u32), 48 MB in all.  Of a longer stream a fixed sample of n_sample records is written, the same in every run, so
+    that the outputs of two builds can be compared reply for reply."""
+    from dint_b200 import wire
+    rec = wire.as_records(wire.FASST, raw)
+    if len(rec) > n_sample:
+        rec = rec[np.sort(np.random.default_rng(0).choice(len(rec), n_sample, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for f in rec.dtype.names:
+        np.save(os.path.join(out_dir, f"lock_fasst_reply_{f}.npy"), rec[f].astype(np.float64))
 
 
-def run_fasst(args, torch, fam_name, fam, steps, warmup, do_e2e=True, do_ref=True, timed_seconds=None):
+def run_fasst(args, torch, fam_name, fam, steps, warmup, do_e2e=True, do_ref=True, dump_dir=None):
     """N = 1.  Returns the result dict main() turns into the JSON line."""
     from dint_b200 import Engine, PinnedBuffer, wire
     from dint_b200.workloads import Workload
-    global TIMED_SECONDS
-    if timed_seconds is not None:
-        saved, TIMED_SECONDS = TIMED_SECONDS, timed_seconds
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", 0)))
     n_steps, msg = steps + warmup, 9
     rq_pin, rs_pin = PinnedBuffer(CLIENTS * msg), PinnedBuffer(CLIENTS * msg)
@@ -215,33 +222,27 @@ def run_fasst(args, torch, fam_name, fam, steps, warmup, do_e2e=True, do_ref=Tru
             eng.submit_tensor(d_req[s], d_out[0])
         torch.cuda.synchronize(dev)
         ok = bool((d_out[0].cpu().numpy() == resps[warmup - 1]).all()) if warmup else True
-        snap = eng.snapshot()                    # the state every cycle starts from
-        ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
-        ev[0].record(stream)
-        for s in range(steps):                   # one untimed cycle: sizes the timed region, warms everything
-            eng.submit_tensor(d_req[warmup + s], d_out[s])
-        ev[1].record(stream)
-        torch.cuda.synchronize(dev)
-        cycles = cycles_for(ev[0].elapsed_time(ev[1]) / steps, steps)
+        snap = eng.snapshot()                    # the state the timed steps start from
         eng.reset_stats()
         eng.profile(Engine.PROF_APPLY)           # events around the dominant kernel only (all-kernel profiling costs ~20 %)
         sampler = ClockSampler(dev.index)
         sampler.start()
         time.sleep(0.01)
         torch.cuda.synchronize(dev)
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
         ev[0].record(stream)
-        for _ in range(cycles):
-            eng.restore(snap, stream.cuda_stream)                # inside the timed region
-            for s in range(steps):
-                eng.submit_tensor(d_req[warmup + s], d_out[s])
+        for s in range(steps):
+            eng.submit_tensor(d_req[warmup + s], d_out[s])
         ev[1].record(stream)
         torch.cuda.synchronize(dev)
         ms = ev[0].elapsed_time(ev[1])
         clocks = sampler.stop()
         eng.profile(False)
+        if dump_dir is not None:
+            dump_replies(dump_dir, d_out[steps - 1].cpu().numpy())
         kt, st = eng.kernel_times(), eng.stats()
         n_bad = sum(0 if bool((d_out[s].cpu().numpy() == resps[warmup + s]).all()) else 1 for s in range(steps))
-        out.update(ms=ms, cycles=cycles, kernel_times=kt, stats=st, clocks=clocks, parity_replay=(ok and n_bad == 0))
+        out.update(ms=ms, kernel_times=kt, stats=st, clocks=clocks, parity_replay=(ok and n_bad == 0))
         # a fully profiled cycle (not the timed one) for the per-kernel breakdown
         eng.reset_stats()
         eng.profile(True)
@@ -253,9 +254,9 @@ def run_fasst(args, torch, fam_name, fam, steps, warmup, do_e2e=True, do_ref=Tru
         out["all_kernel_times"] = eng.kernel_times()
         eng.free_snapshot(snap)
         del d_req, d_out
-    out.update(committed=sum(committed[warmup:]) * cycles, requests=steps * STEP_REQS * cycles, steps_timed=steps * cycles)
+    out.update(committed=sum(committed[warmup:]), requests=steps * STEP_REQS, steps_timed=steps)
     alg, mix = fasst_alg_bytes(resps[warmup:])
-    out.update(alg_bytes=alg * cycles, reply_mix=mix)
+    out.update(alg_bytes=alg, reply_mix=mix)
     # ---- end to end through the host-facing C ABI call (pinned host buffers, H2D + D2H inside) ----
     if do_e2e:
         with Engine(wire.FASST, device=dev.index, chunk=args.chunk) as eng:
@@ -266,24 +267,16 @@ def run_fasst(args, torch, fam_name, fam, steps, warmup, do_e2e=True, do_ref=Tru
                 eng.submit(host_in[0].array, out=host_out.array)
             for s in range(steps):
                 host_in[s].array[:] = reqs[warmup + s]              # staging into pinned memory: not timed
-            snap = eng.snapshot()
-            t_e2e, n_e2e, ok2 = 0.0, 0, True
-            while t_e2e < TIMED_SECONDS:
-                eng.restore(snap, 0)
-                torch.cuda.synchronize(dev)
-                for s in range(steps):
-                    t0 = time.perf_counter()
-                    eng.submit(host_in[s].array, out=host_out.array)   # timed: H2D + kernels + D2H, returns when resp is complete
-                    t_e2e += time.perf_counter() - t0
-                    n_e2e += 1
-                ok2 = ok2 and bool((host_out.array == resps[n_steps - 1]).all())
-            eng.free_snapshot(snap)
-            out.update(e2e_s=t_e2e, e2e_steps=n_e2e, e2e_parity=ok2,
-                       e2e_committed=sum(committed[warmup:]) * (n_e2e // steps), e2e_requests=STEP_REQS * n_e2e)
+            torch.cuda.synchronize(dev)
+            t_e2e = 0.0
+            for s in range(steps):
+                t0 = time.perf_counter()
+                eng.submit(host_in[s].array, out=host_out.array)   # timed: H2D + kernels + D2H, returns when resp is complete
+                t_e2e += time.perf_counter() - t0
+            out.update(e2e_s=t_e2e, e2e_steps=steps, e2e_parity=bool((host_out.array == resps[n_steps - 1]).all()),
+                       e2e_committed=sum(committed[warmup:]), e2e_requests=STEP_REQS * steps)
     if ref_bg is not None:
         out["cpu_baseline"] = ref_bg.get(timeout=600)
-    if timed_seconds is not None:
-        TIMED_SECONDS = saved
     out["first_step"] = (reqs[0], resps[0], txn_per_req)
     return out
 
@@ -297,7 +290,7 @@ def gather_prefix(torch, dist, rank, world, arr):
     return [p.cpu().numpy() for p in parts] if rank == 0 else None
 
 
-def run_fasst_sharded(args, torch, dist, rank, world, scaled, steps, warmup, do_e2e=True):
+def run_fasst_sharded(args, torch, dist, rank, world, scaled, steps, warmup, do_e2e=True, dump_dir=None):
     """Every rank drives its own 1,048,576 clients; requests are routed to the owning shard through the library's
     dispatch / engine / combine step over NVLink peer memory (dint_shard_submit_many).  scaled=True: the key space
     grows with the GPU count (36 M slots and 24 M ids per GPU: the per-GPU state and the contention stay what they are
@@ -353,44 +346,33 @@ def run_fasst_sharded(args, torch, dist, rank, world, scaled, steps, warmup, do_
     for s in range(warmup):
         step(s, 0)
     torch.cuda.synchronize(dev)
-    dist.barrier()
-    snap = se.engine.snapshot()
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
-    ev[0].record(stream)
-    for s in range(steps):
-        step(warmup + s, s)
-    ev[1].record(stream)
-    torch.cuda.synchronize(dev)
-    t = torch.tensor([ev[0].elapsed_time(ev[1]) / steps], device=dev, dtype=torch.float64)
-    dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    cycles = cycles_for(float(t[0]), steps)
     se.engine.reset_stats()
     se.engine.profile(se.engine.PROF_APPLY)
     sampler = ClockSampler(dev.index)
     sampler.start()
     dist.barrier()
     torch.cuda.synchronize(dev)
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     ev[0].record(stream)
-    for _ in range(cycles):
-        se.engine.restore(snap, stream.cuda_stream)          # local state, ordered on the engine's stream between two batches
-        for s in range(steps):
-            step(warmup + s, s)
+    for s in range(steps):
+        step(warmup + s, s)
     ev[1].record(stream)
     torch.cuda.synchronize(dev)
     dist.barrier()
     ms = ev[0].elapsed_time(ev[1])
     clocks = sampler.stop()
     se.engine.profile(False)
+    if dump_dir is not None and rank == 0:
+        dump_replies(dump_dir, torch.cat(last[steps - 1]).cpu().numpy())
     n_bad = 0
     for s in range(steps):
         got = torch.cat(last[s]).cpu().numpy()
         n_bad += 0 if bool((got == resps[warmup + s]).all()) else 1
     ok = n_bad == 0 and se.check_p2p() == (0, 0) and flags_rec == (0, 0)
-    out = dict(ms=ms, cycles=cycles, kernel_times=se.engine.kernel_times(), stats=se.engine.stats(), clocks=clocks, parity_replay=ok,
-               committed=sum(committed[warmup:]) * cycles, requests=steps * STEP_REQS * cycles, steps_timed=steps * cycles, wl_stats=wl_stats)
+    out = dict(ms=ms, kernel_times=se.engine.kernel_times(), stats=se.engine.stats(), clocks=clocks, parity_replay=ok,
+               committed=sum(committed[warmup:]), requests=steps * STEP_REQS, steps_timed=steps, wl_stats=wl_stats)
     alg, mix = fasst_alg_bytes(resps[warmup:])
-    out.update(alg_bytes=alg * cycles, reply_mix=mix)
-    se.engine.free_snapshot(snap)
+    out.update(alg_bytes=alg, reply_mix=mix)
     se.close()
     del d_req
     # ---- end to end: pinned host -> H2D | dispatch | engine | combine | D2H (dint_shard_submit_host), per step ----
@@ -402,28 +384,15 @@ def run_fasst_sharded(args, torch, dist, rank, world, scaled, steps, warmup, do_
         rounds = lambda p: [p[r * rb:(r + 1) * rb] for r in range(ROUNDS_PER_STEP)]
         for s in range(warmup):
             se.submit_many_host(rounds(pin_w[s]), rounds(pin_out))
-        snap = se.engine.snapshot()
-        t_e2e, n_e2e, ok2 = 0.0, 0, True
-        go = torch.ones(1, device=dev)
-        while True:
-            se.engine.restore(snap, 0)
+        t_e2e = 0.0
+        for s in range(steps):
+            dist.barrier()
             torch.cuda.synchronize(dev)
-            for s in range(steps):
-                dist.barrier()
-                torch.cuda.synchronize(dev)
-                t0 = time.perf_counter()
-                se.submit_many_host(rounds(pin_in[s]), rounds(pin_out))
-                t_e2e += time.perf_counter() - t0
-                n_e2e += 1
-            ok2 = ok2 and bool((pin_out.numpy() == resps[n_steps - 1]).all())
-            go[0] = 1.0 if t_e2e < TIMED_SECONDS else 0.0       # all ranks stop together
-            dist.all_reduce(go, op=dist.ReduceOp.MAX)
-            if float(go[0]) == 0.0:
-                break
-        ok2 = ok2 and se.check_p2p() == (0, 0)
-        se.engine.free_snapshot(snap)
-        out.update(e2e_s=t_e2e, e2e_steps=n_e2e, e2e_parity=ok2, e2e_committed=sum(committed[warmup:]) * (n_e2e // steps),
-                   e2e_requests=STEP_REQS * n_e2e)
+            t0 = time.perf_counter()
+            se.submit_many_host(rounds(pin_in[s]), rounds(pin_out))
+            t_e2e += time.perf_counter() - t0
+        ok2 = bool((pin_out.numpy() == resps[n_steps - 1]).all()) and se.check_p2p() == (0, 0)
+        out.update(e2e_s=t_e2e, e2e_steps=steps, e2e_parity=ok2, e2e_committed=sum(committed[warmup:]), e2e_requests=STEP_REQS * steps)
         se.close()
     if par_bg is not None:
         out["oracle_parity"] = par_bg.get(timeout=900)
@@ -895,6 +864,8 @@ def main():
     ap.add_argument("--impl", default="dint_b200", choices=["dint_b200", "reference"])
     ap.add_argument("--chunk", type=int, default=1 << 20)
     ap.add_argument("--no-extra", action="store_true", help="skip the side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the replies of the last timed step to DIR/*.npy (float64; at N > 1 rank 0's)")
     ap.add_argument("--extra-only", default=None, help=argparse.SUPPRESS)     # child-process mode for a side measurement
     args = ap.parse_args()
     if args.extra_only:
@@ -925,9 +896,9 @@ def main():
 
     t_start = time.time()
     if world > 1:
-        res = run_fasst_sharded(args, torch, dist, rank, world, True, args.steps, args.warmup)
+        res = run_fasst_sharded(args, torch, dist, rank, world, True, args.steps, args.warmup, dump_dir=args.dump_outputs)
     else:
-        res = run_fasst(args, torch, "REF", REF, args.steps, args.warmup)
+        res = run_fasst(args, torch, "REF", REF, args.steps, args.warmup, dump_dir=args.dump_outputs)
 
     # reduce over ranks: time = max, work = sum
     ms, committed, reqs = res["ms"], res["committed"], res["requests"]
@@ -1004,7 +975,7 @@ def main():
             "all_kernels_ms_profiled_cycle": {k: round(v[1], 3) for k, v in akt.items()}}
     if "k_classify" in akt:
         l1, t1 = akt["k_classify"]
-        ach1 = (res["alg_bytes"] / res["cycles"]) / max(1, l1) / (t1 / l1 * 1e-3) / 1e9 if world == 1 else None
+        ach1 = res["alg_bytes"] / max(1, l1) / (t1 / l1 * 1e-3) / 1e9 if world == 1 else None
         roof["k_classify"] = {"avg_launch_us": t1 / l1 * 1e3, "launches_profiled_cycle": l1,
                               "achieved_same_algorithmic_bytes": ach1, "frac": (ach1 / peak) if ach1 else None,
                               "note": "second pass over the same requests (conflict flags + replay of the previous chunk): it moves no algorithmic byte "
@@ -1020,8 +991,7 @@ def main():
                                       "uniform lock ids (BASELINE.md section 1 note, lock_fasst/caladan/trace_init.sh:9-27): the headline "
                                       "runs that reference shape; the literal reading (4800 ids, Zipf 0.8) is extra.lock_fasst_HOT",
                    "requests_per_step": STEP_REQS * world, "chunk": args.chunk,
-                   "timed_region": f"{res['cycles']} cycles x {args.steps} recorded steps = {res['steps_timed']} steps, {ms * 1e-3:.3f} s; the server state is "
-                                   "restored from a snapshot at the start of every cycle INSIDE the timed region",
+                   "timed_region": f"{res['steps_timed']} recorded steps once, {ms * 1e-3:.3f} s, from the server state the warm-up steps left",
                    "cache": "every step replays a different 37.7 MB trace segment (K segments larger than L2; lock/version tables 148.5 MB > 126 MB L2)",
                    "parallelism": (f"key-space sharded x{world}: dispatch / engine / combine kernels over NVLink peer memory (owner = slot % {world}), "
                                    "one process per GPU") if world > 1 else "single GPU"},
@@ -1059,7 +1029,7 @@ def main():
         line["cpu_baseline"].pop("gpu_replies_equal_reference", None)
     if not args.no_extra and world == 1:
         try:
-            hot = run_fasst(args, torch, "HOT", HOT, max(3, args.steps // 3), 3, do_e2e=False, do_ref=True, timed_seconds=min(TIMED_SECONDS, 0.5))
+            hot = run_fasst(args, torch, "HOT", HOT, max(3, args.steps // 3), 3, do_e2e=False, do_ref=True)
             extra["lock_fasst_HOT"] = {
                 "workload": "BASELINE.json literal: 4800 lock ids, Zipf 0.8, same clients/protocol",
                 "txn_per_s": hot["committed"] / (hot["ms"] * 1e-3), "requests_per_s": hot["requests"] / (hot["ms"] * 1e-3),

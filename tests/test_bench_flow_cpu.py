@@ -17,7 +17,7 @@ HARNESS = textwrap.dedent('''
     torch.cuda.is_available = lambda: True
     torch.cuda.empty_cache = lambda: None
     import bench as B
-    res = dict(ms=1113.0, cycles=10, kernel_times={"k_apply": (160, 5.0)}, stats={"kernel_launches": 500, "conflicted": 10, "requests": 1000},
+    res = dict(ms=1113.0, kernel_times={"k_apply": (160, 5.0)}, stats={"kernel_launches": 500, "conflicted": 10, "requests": 1000},
                clocks={"sm_mhz": 1965, "sm_max_mhz": 1965, "reasons": [], "samples": 5}, parity_replay=True,
                all_kernel_times={"k_classify": (40, 1.06), "k_apply": (40, 1.25), "k_ordered": (40, 0.2)}, committed=650000000, requests=16000000000,
                steps_timed=40, alg_bytes=3.8e9, reply_mix={}, e2e_s=1.0, e2e_steps=40, e2e_parity=True, e2e_committed=150000000, e2e_requests=4000000000,
@@ -66,3 +66,27 @@ def test_bench_watchdog_prints_the_headline_when_the_extras_hang():
     for k in KEYS:
         assert k in d, k
     assert "exceeded their deadline" in d["note"] and "extra" not in d
+
+
+def test_dump_outputs_write_a_fixed_exact_sample_of_the_replies(tmp_path):
+    import numpy as np
+    import bench as B
+    from dint_b200 import wire
+    rec = np.zeros(B.STEP_REQS, dtype=wire.MSG_DTYPE[wire.FASST])
+    idx = np.arange(rec.size, dtype=np.uint64)
+    rec["type"] = 4 + idx % 5
+    rec["lid"] = idx
+    rec["ver"] = (idx * 2654435761) % 2**32
+    for d in ("a", "b"):
+        B.dump_replies(str(tmp_path / d), wire.as_bytes(rec))
+    names = ["lock_fasst_reply_lid.npy", "lock_fasst_reply_type.npy", "lock_fasst_reply_ver.npy"]
+    assert sorted(p.name for p in (tmp_path / "a").iterdir()) == names
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 << 20
+    got = {}
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float64 and np.array_equal(a, b)         # the same sample in every run
+        got[n.split("_")[-1][:-4]] = a.astype(np.uint64)
+    lid = got["lid"]
+    assert 0 < lid.size < rec.size and (np.diff(lid) > 0).all()
+    assert np.array_equal(got["type"], 4 + lid % 5) and np.array_equal(got["ver"], (lid * 2654435761) % 2**32)

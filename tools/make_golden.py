@@ -17,6 +17,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+import golden_util as G         # noqa: E402
 import oracle_lib as O          # noqa: E402
 import trace_gen as T           # noqa: E402
 from dint_b200 import wire      # noqa: E402
@@ -79,6 +80,11 @@ def main():
             shard0.append(rq.reshape(-1, wire.MSG_SIZE[kind])[dst == 0].reshape(-1).copy())
             wl.feed(cl.submit(rq, dst))
         save(name, kind, np.concatenate(shard0), cfg)
+    # seeded trace_gen traces, replies only (golden_util.TRACES)
+    for name, (kind, make) in G.TRACES.items():
+        req = make()
+        G.save_trace(name, req, O.run_ref(kind, req)[0])
+        print(f"trace_gen/{name}: {req.size // wire.MSG_SIZE[kind]} requests")
 
 
 if __name__ == "__main__":
