@@ -371,6 +371,7 @@ static int pull_counters(dint_engine* e) {
   e->stats.errors = h[0];
   e->stats.conflicted = h[1];
   e->stats.max_run = h[2];
+  e->stats.fallback_chunks = h[3];
   return DINT_OK;
 }
 
@@ -936,6 +937,7 @@ int dint_submit(dint_engine* e, const void* req, uint64_t n, void* resp) {
   e->stats.errors = e->h_counters[0];
   e->stats.conflicted = e->h_counters[1];
   e->stats.max_run = e->h_counters[2];
+  e->stats.fallback_chunks = e->h_counters[3];
   return e->stats.errors != err_before ? DINT_EPROTO : DINT_OK;
 }
 

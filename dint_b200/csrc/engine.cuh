@@ -133,7 +133,7 @@ struct Ctx {
   unsigned long long* log_tilebase;  // [n_tiles] absolute append ordinal of the tile's first append (K1b)
   unsigned long long* log_total;     // [2]: [0] appends before this chunk ... running total, [1] this chunk's total
   // bookkeeping
-  unsigned long long* counters;   // [0] errors [1] conflicted [2] max_run
+  unsigned long long* counters;   // [0] errors [1] conflicted [2] max_run [3] chunks replayed by the radix fallback
   uint32_t* gbar;                 // k_ordered's grid barrier when it is not launched cooperatively
   uint32_t coop_launch;           // 1: k_ordered was launched cooperatively
   // where the replies go.  Default: `resp`, one contiguous array.  Inside the multi-GPU step the batch is W source

@@ -626,15 +626,17 @@ DINT_D void ordered_buckets(const Ctx& c, uint8_t* scratch) {
 // (lock_fasst/udp/server.cc:86-114).  Such maps compose associatively, so the state every request of a run
 // SEES is an exclusive segmented scan over the sorted list -- a run of tens of thousands of requests on one
 // hot slot (HOT: 4800 ids, Zipf) is then replayed by the whole grid instead of by one thread.
-// Encoding: bits 0-31 d, bits 32-33 lock map (0 id, 1 set 0, 2 set 1), bit 34 segment head.
+// Encoding: bits 0-31 d, bits 32-33 lock map (0 id, 1 set 0, 2 set 1), bit 34 segment head, bits 35-63 the number
+// of requests composed since the segment head (so the inclusive value at a run's last entry holds the run length;
+// exact for runs shorter than 2^29 requests, so for chunks of up to 2^29).
 DINT_D uint64_t fx_of(uint32_t type, bool head) {
   const uint64_t lt = (type == 0) ? 0ull : (type == 1) ? 2ull : 1ull;
-  return (uint64_t)(type == 3 ? 1u : 0u) | (lt << 32) | ((uint64_t)(head ? 1u : 0u) << 34);
+  return (uint64_t)(type == 3 ? 1u : 0u) | (lt << 32) | ((uint64_t)(head ? 1u : 0u) << 34) | (1ull << 35);
 }
 DINT_D uint64_t fx_compose(uint64_t a, uint64_t b) {        // a then b, segment-aware
   if ((b >> 34) & 1ull) return b;
   const uint64_t lt = ((b >> 32) & 3ull) ? ((b >> 32) & 3ull) : ((a >> 32) & 3ull);
-  return (uint64_t)((uint32_t)a + (uint32_t)b) | (lt << 32) | (a & (1ull << 34));
+  return (uint64_t)((uint32_t)a + (uint32_t)b) | (lt << 32) | (a & (1ull << 34)) | (((a >> 35) + (b >> 35)) << 35);
 }
 constexpr uint64_t kFxId = 0ull;
 
@@ -913,6 +915,7 @@ __global__ void __launch_bounds__(kThreads) k_ordered(const Ctx c) {
       }
       grid.sync();
       // (3) replies: every entry derives the state it sees from its exclusive prefix
+      uint32_t run_max = 0;                                    // longest run ending in this thread's entries
       for (uint32_t T = blockIdx.x; T < n_st; T += gridDim.x) {
         uint64_t f[kSortItems]; uint32_t ty[kSortItems]; uint32_t cnt;
         load8(T, f, ty, cnt);
@@ -957,9 +960,12 @@ __global__ void __launch_bounds__(kThreads) k_ordered(const Ctx c) {
             const bool last = p + 1 == nc || (uint32_t)(src[p + 1] >> 32) != g;
             if (last) dst[p] = (uint64_t)st.ver | ((uint64_t)st.lock << 32) | ((uint64_t)(st.dirty_ver ? 1u : 0u) << 33);
             pre = head ? f[k] : fx_compose(pre, f[k]);
+            if (last) run_max = max(run_max, (uint32_t)(pre >> 35));   // inclusive prefix of a run's last entry: its length
           }
         }
       }
+      run_max = __reduce_max_sync(0xffffffffu, run_max);        // the loop above is uniform per CTA: every lane is here
+      if (lane_id() == 0 && run_max > 1) atomicMax(&c.counters[2], (unsigned long long)run_max);
       grid.sync();
       // (4) final state of every run
       for (uint32_t p = blockIdx.x * kThreads + tid; p < nc; p += gridDim.x * kThreads) {
@@ -998,7 +1004,10 @@ __global__ void __launch_bounds__(kThreads) k_ordered(const Ctx c) {
         if (p == 0 || (uint32_t)(src[p - 1] >> 32) != (uint32_t)(src[p] >> 32)) replay_run<KIND>(c, src, p, nc);
     }
   }
-  if (blockIdx.x == 0 && tid == 0) atomicAdd(&c.counters[1], (unsigned long long)nc);
+  if (blockIdx.x == 0 && tid == 0) {
+    atomicAdd(&c.counters[1], (unsigned long long)nc);
+    atomicAdd(&c.counters[3], 1ull);                   // chunks that took this fallback
+  }
 }
 
 }  // namespace dint

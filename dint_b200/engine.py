@@ -26,7 +26,8 @@ class DintCfg(C.Structure):
 class DintStats(C.Structure):
     _fields_ = [("requests", C.c_uint64), ("chunks", C.c_uint64), ("kernel_launches", C.c_uint64),
                 ("conflicted", C.c_uint64), ("max_run", C.c_uint64), ("errors", C.c_uint64),
-                ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("kv_rebuilds", C.c_uint64), ("reserved", C.c_uint64 * 3)]
+                ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("kv_rebuilds", C.c_uint64),
+                ("fallback_chunks", C.c_uint64), ("reserved", C.c_uint64 * 2)]
 
 
 class DintPeerPtrs(C.Structure):

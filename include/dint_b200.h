@@ -90,7 +90,9 @@ typedef struct dint_stats {
   uint64_t h2d_bytes, d2h_bytes;
   uint64_t kv_rebuilds;     /* KV tables rehashed to reclaim tombstones (the reference frees entries on delete:
                                store/udp/kvs.h:124-133) */
-  uint64_t reserved[3];
+  uint64_t fallback_chunks; /* chunks whose listed requests overflowed a replay bucket and were replayed by the
+                               radix-sort fallback instead */
+  uint64_t reserved[2];
 } dint_stats;
 
 /* Per-kernel device time, accumulated with CUDA events while profiling is on. */

@@ -95,3 +95,9 @@ def test_udp_front_end_builds_and_fails_loudly_without_a_gpu():
     r = subprocess.run([_build.UDP_SERVER, "lock_fasst", "--port", "29731"], capture_output=True, timeout=60)
     assert r.returncode == 1 and b"dint_create failed" in r.stderr
     assert subprocess.run([_build.UDP_SERVER, "no_such_server"], capture_output=True, timeout=60).returncode == 2
+
+
+def test_stats_struct_layout():
+    """dint_stats is 12 u64 wide; fallback_chunks took the first reserved slot, so the layout did not move."""
+    assert C.sizeof(E.DintStats) == 12 * 8
+    assert E.DintStats.kv_rebuilds.offset == 8 * 8 and E.DintStats.fallback_chunks.offset == 9 * 8

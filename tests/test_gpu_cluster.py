@@ -128,14 +128,17 @@ def test_cluster_serves_client_chosen_shards(kind, n, clients, G):
 def test_cluster_from_c():
     """A plain C caller (gcc, no Python, no torch): tests/c/cluster_check.c links libdint_b200.so and the oracle and
     compares dint_cluster_submit with ONE sequential server for lock_fasst (3 shards) and with 3 shard servers for
-    smallbank -- the call sequence a C/C++ transport front-end makes (INTEGRATION.md)."""
+    smallbank -- the call sequence a C/C++ transport front-end makes (INTEGRATION.md).  The program is built in a
+    temporary directory, so the test writes nothing into the source tree (which may be read-only or another user's)."""
+    import tempfile
     from dint_b200 import _build
-    exe = os.path.join(ROOT, "tests", "c", "cluster_check")
     src = os.path.join(ROOT, "tests", "c", "cluster_check.c")
-    subprocess.run(["gcc", "-O2", "-Wall", "-o", exe, src, "-I" + os.path.join(ROOT, "include"), "-I" + os.path.join(ROOT, "oracle"),
-                    "-L" + _build.LIBDIR, "-ldint_b200", "-L" + os.path.join(ROOT, "oracle"), "-ldint_oracle",
-                    "-Wl,-rpath," + _build.LIBDIR, "-Wl,-rpath," + os.path.join(ROOT, "oracle")], check=True)
-    r = subprocess.run([exe], capture_output=True, timeout=300)
+    with tempfile.TemporaryDirectory() as td:
+        exe = os.path.join(td, "cluster_check")
+        subprocess.run(["gcc", "-O2", "-Wall", "-o", exe, src, "-I" + os.path.join(ROOT, "include"), "-I" + os.path.join(ROOT, "oracle"),
+                        "-L" + _build.LIBDIR, "-ldint_b200", "-L" + os.path.join(ROOT, "oracle"), "-ldint_oracle",
+                        "-Wl,-rpath," + _build.LIBDIR, "-Wl,-rpath," + os.path.join(ROOT, "oracle")], check=True)
+        r = subprocess.run([exe], capture_output=True, timeout=300)
     sys.stdout.write(r.stdout.decode())
     assert r.returncode == 0, r.stdout.decode() + r.stderr.decode()
     assert b"cluster_check: OK" in r.stdout
