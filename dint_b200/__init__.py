@@ -5,6 +5,6 @@
     resp = eng.submit(requests)         # packed wire structs in, packed wire structs out
 """
 from . import wire
-from .engine import Engine, GpuCluster, GpuClients, PinnedBuffer, DintError, default_cfg, lib
+from .engine import Engine, GpuCluster, GpuClients, GpuTxnClients, PinnedBuffer, DintError, default_cfg, lib
 
-__all__ = ["Engine", "GpuCluster", "GpuClients", "PinnedBuffer", "DintError", "default_cfg", "lib", "wire"]
+__all__ = ["Engine", "GpuCluster", "GpuClients", "GpuTxnClients", "PinnedBuffer", "DintError", "default_cfg", "lib", "wire"]

@@ -15,6 +15,7 @@
 #include "route.cuh"
 #include "kv.cuh"
 #include "clients.cuh"
+#include "txn_clients.cuh"
 
 using namespace dint;
 
@@ -1822,6 +1823,191 @@ int dint_clients_peek(dint_clients* c, void* next_req_host, void* last_resp_host
   }
   if (next_req_host) CU(cudaMemcpy(next_req_host, c->req, (size_t)c->cc.n_clients * 9, cudaMemcpyDeviceToHost));
   if (last_resp_host) CU(cudaMemcpy(last_resp_host, c->resp, (size_t)c->cc.n_clients * 9, cudaMemcpyDeviceToHost));
+  return DINT_OK;
+}
+
+}  // extern "C"
+
+extern "C" {
+// ---- TATP / SmallBank closed-loop clients on the GPU (txn_clients.cuh) -------------------------------------------------
+struct dint_txn_clients {
+  std::vector<dint_engine*> eng;
+  int kind = 0, device = 0;
+  uint32_t G = 0, msz = 0;
+  TxnDevCtx x{};
+  int p = 0;                          // parity of the round whose requests are pending
+  uint32_t* h_tot = nullptr;          // pinned copy of x.tot
+  uint32_t tot[8] = {0}, tot_prev[8] = {0};
+  bool served = false;                // a round has been served: last replies exist
+  uint64_t st_requests = 0, st_rounds = 0;
+  cudaEvent_t ev = nullptr;
+  std::vector<void*> allocs;
+};
+
+void dint_txn_clients_destroy(dint_txn_clients* c) {
+  if (!c) return;
+  cudaSetDevice(c->device);
+  cudaDeviceSynchronize();
+  for (void* q : c->allocs) cudaFree(q);
+  if (c->h_tot) cudaFreeHost(c->h_tot);
+  if (c->ev) cudaEventDestroy(c->ev);
+  delete c;
+}
+
+// k_txn_step (absorb or begin, then count) + k_txn_scan + k_txn_emit for parity p, then the per-shard totals to the host
+static int txn_clients_round(dint_txn_clients* c, int init, cudaStream_t s) {
+  const TxnDevCtx& x = c->x;
+  if (c->kind == DINT_TATP) k_txn_step<DINT_TATP><<<x.nb, kTxnThreads, 0, s>>>(x, init, c->p);
+  else k_txn_step<DINT_SMALLBANK><<<x.nb, kTxnThreads, 0, s>>>(x, init, c->p);
+  k_txn_scan<<<c->G, kTxnScanThreads, 0, s>>>(x, c->p);
+  if (c->kind == DINT_TATP) k_txn_emit<DINT_TATP><<<x.nb, kTxnThreads, 0, s>>>(x, c->p);
+  else k_txn_emit<DINT_SMALLBANK><<<x.nb, kTxnThreads, 0, s>>>(x, c->p);
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(c->h_tot, x.tot, 9 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  CU(cudaEventRecord(c->ev, s));
+  CU(cudaEventSynchronize(c->ev));
+  if (c->h_tot[8]) return set_err(DINT_EIO, "a client sent one shard more records in one round than the buffers are sized for");
+  memcpy(c->tot_prev, c->tot, sizeof c->tot);
+  for (uint32_t s_ = 0; s_ < c->G; s_++) c->tot[s_] = c->h_tot[s_];
+  return DINT_OK;
+}
+
+int dint_txn_clients_create(dint_engine* const* shards, uint32_t n_shards, uint32_t n_clients, uint32_t gid0, uint32_t subscribers,
+                            dint_txn_clients** out) {
+  if (!shards || !out) return set_err(DINT_EINVAL, "null argument");
+  *out = nullptr;
+  if (n_shards == 0 || n_shards == 2 || n_shards > 8) return set_err(DINT_EINVAL, "n_shards must be 1 or 3..8 (primary + 2 distinct backups)");
+  if (n_clients == 0 || n_clients > (1u << 26)) return set_err(DINT_EINVAL, "n_clients must be 1..2^26");
+  if (subscribers < 3) return set_err(DINT_EINVAL, "subscribers / accounts must be >= 3");
+  for (uint32_t i = 0; i < n_shards; i++) {
+    const dint_engine* e = shards[i];
+    if (!e) return set_err(DINT_EINVAL, "null engine");
+    if ((e->kind != DINT_TATP && e->kind != DINT_SMALLBANK) || e->kind != shards[0]->kind)
+      return set_err(DINT_EINVAL, "the engines must all be tatp or all smallbank");
+    if (e->device != shards[0]->device) return set_err(DINT_EINVAL, "the engines must all be on one device");
+    if (n_shards > 3 && (e->cfg.txn_shards != n_shards || e->cfg.txn_shard_id != i))
+      return set_err(DINT_EINVAL, "with more than 3 shards, engine i must be configured as shard i of n_shards (txn_shards / txn_shard_id)");
+  }
+  dint_txn_clients* c = new dint_txn_clients();
+  c->eng.assign(shards, shards + n_shards);
+  c->kind = shards[0]->kind; c->device = shards[0]->device; c->G = n_shards; c->msz = kMsgSize[c->kind];
+  TxnDevCtx& x = c->x;
+  x.P.G = n_shards; x.P.subscribers = subscribers; x.P.accounts = subscribers; x.P.hot = txn::sb_hot_accounts(subscribers);
+  x.n_clients = n_clients; x.nb = (n_clients + kTxnThreads - 1) / kTxnThreads; x.gid0 = gid0;
+  x.bound = txn::max_per_shard(c->kind, n_shards);
+  const size_t n = n_clients, G = n_shards;
+  int rc = DINT_OK;
+  auto alloc = [&](void** q, size_t bytes) {
+    if (rc) return;
+    cudaError_t ce = cudaMalloc(q, bytes);           // 256-byte aligned: the engines need 16
+    if (ce != cudaSuccess) { *q = nullptr; rc = set_err(DINT_ENOMEM, "client state", ce); return; }
+    c->allocs.push_back(*q);
+  };
+  if (cudaSetDevice(c->device) != cudaSuccess) { delete c; return set_err(DINT_EIO, "cudaSetDevice", cudaGetLastError()); }
+  alloc(&x.cl, n * (c->kind == DINT_TATP ? sizeof(txn::TatpClient) : sizeof(txn::SbClient)));
+  for (uint32_t s = 0; s < n_shards; s++) {
+    alloc((void**)&x.req[s], n * x.bound * c->msz + 16);
+    alloc((void**)&x.resp[s], n * x.bound * c->msz + 16);
+  }
+  for (int q = 0; q < 2; q++) {
+    alloc((void**)&x.loff[q], G * n * 4);
+    alloc((void**)&x.base[q], G * x.nb * 4);
+    alloc((void**)&x.route[q], n * 4);
+  }
+  alloc((void**)&x.ctatot, G * x.nb * 4);
+  alloc((void**)&x.tot, 16 * 4);
+  alloc((void**)&x.stats, 18 * sizeof(unsigned long long));
+  if (!rc && cudaMallocHost((void**)&c->h_tot, 16 * 4) != cudaSuccess) rc = set_err(DINT_ENOMEM, "pinned totals", cudaGetLastError());
+  if (!rc && cudaEventCreateWithFlags(&c->ev, cudaEventDisableTiming) != cudaSuccess) rc = set_err(DINT_EIO, "event", cudaGetLastError());
+  if (!rc && (cudaMemset(x.tot, 0, 16 * 4) != cudaSuccess || cudaMemset(x.stats, 0, 18 * sizeof(unsigned long long)) != cudaSuccess))
+    rc = set_err(DINT_EIO, "cudaMemset", cudaGetLastError());
+  // every client begins its first transaction; the first round's records go to the shard buffers
+  if (!rc) rc = txn_clients_round(c, 1, nullptr);
+  if (rc) { dint_txn_clients_destroy(c); return rc; }
+  *out = c;
+  return DINT_OK;
+}
+
+// `rounds` rounds on cuda_stream: serve the pending records with the shard engines, then absorb + count, scan, emit.
+// Returns after the last round's totals reached the host (each round synchronises once on them).
+int dint_txn_clients_run(dint_txn_clients* c, uint32_t rounds, void* cuda_stream) {
+  if (!c) return set_err(DINT_EINVAL, "null argument");
+  CU(cudaSetDevice(c->device));
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  for (uint32_t r = 0; r < rounds; r++) {
+    for (uint32_t i = 0; i < c->G; i++) {
+      if (!c->tot[i]) continue;                            // as Cluster.submit: an empty shard is not called
+      int rc = run_device(c->eng[i], c->x.req[i], c->tot[i], c->x.resp[i], s);
+      if (rc) return rc;
+      c->st_requests += c->tot[i];
+    }
+    c->st_rounds++;
+    c->served = true;
+    c->p ^= 1;
+    int rc = txn_clients_round(c, 0, s);
+    if (rc) return rc;
+  }
+  return DINT_OK;
+}
+
+// out: requests served, transactions begun, committed, rounds, begun by type[7], committed by type[7] (synchronises)
+int dint_txn_clients_stats(dint_txn_clients* c, uint64_t out[18]) {
+  if (!c || !out) return set_err(DINT_EINVAL, "null argument");
+  CU(cudaSetDevice(c->device));
+  CU(cudaDeviceSynchronize());
+  unsigned long long h[18];
+  CU(cudaMemcpy(h, c->x.stats, sizeof h, cudaMemcpyDeviceToHost));
+  for (int i = 0; i < 18; i++) out[i] = h[i];
+  out[0] = c->st_requests;
+  out[3] = c->st_rounds;
+  return DINT_OK;
+}
+
+// rebuild one round in client order (each client's records contiguous, in push order) from the shard buffers
+static int txn_clients_gather(dint_txn_clients* c, int p, uint8_t* const* bufs, const uint32_t* tot, uint8_t* out, uint8_t* dst) {
+  const size_t n = c->x.n_clients, G = c->G, nb = c->x.nb, msz = c->msz;
+  std::vector<uint32_t> route(n), loff(G * n), base(G * nb);
+  std::vector<std::vector<uint8_t>> recs(G);
+  CU(cudaMemcpy(route.data(), c->x.route[p], n * 4, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(loff.data(), c->x.loff[p], G * n * 4, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(base.data(), c->x.base[p], G * nb * 4, cudaMemcpyDeviceToHost));
+  for (size_t s = 0; s < G; s++) {
+    recs[s].resize((size_t)tot[s] * msz);
+    if (tot[s]) CU(cudaMemcpy(recs[s].data(), bufs[s], (size_t)tot[s] * msz, cudaMemcpyDeviceToHost));
+  }
+  size_t j = 0;
+  for (size_t cl = 0; cl < n; cl++) {
+    const uint32_t r = route[cl];
+    uint32_t k[8] = {0};
+    for (uint32_t i = 0; i < (r & 15u); i++, j++) {
+      const uint32_t s = (r >> (4 + 3 * i)) & 7u;
+      const size_t slot = (size_t)base[s * nb + cl / kTxnThreads] + loff[s * n + cl] + k[s]++;
+      if (slot >= tot[s]) return set_err(DINT_EIO, "peek: inconsistent offsets");
+      if (out) memcpy(out + j * msz, recs[s].data() + slot * msz, msz);
+      if (dst) dst[j] = (uint8_t)s;
+    }
+  }
+  return DINT_OK;
+}
+
+// test hook: the pending round's requests + destination shards and the last round's replies, in client order, as
+// dint_txn_next / dint_txn_feed lay them out.  n_out = {records pending, replies of the last round}; pass NULL buffers to
+// learn the sizes first.
+int dint_txn_clients_peek(dint_txn_clients* c, void* next_req_host, uint8_t* next_dst_host, void* last_resp_host, uint64_t n_out[2]) {
+  if (!c) return set_err(DINT_EINVAL, "null argument");
+  CU(cudaSetDevice(c->device));
+  CU(cudaDeviceSynchronize());
+  uint64_t a = 0, b = 0;
+  for (uint32_t s = 0; s < c->G; s++) { a += c->tot[s]; b += c->served ? c->tot_prev[s] : 0; }
+  if (n_out) { n_out[0] = a; n_out[1] = b; }
+  if (next_req_host || next_dst_host) {
+    int rc = txn_clients_gather(c, c->p, c->x.req, c->tot, (uint8_t*)next_req_host, next_dst_host);
+    if (rc) return rc;
+  }
+  if (last_resp_host && c->served) {
+    int rc = txn_clients_gather(c, c->p ^ 1, c->x.resp, c->tot_prev, (uint8_t*)last_resp_host, nullptr);
+    if (rc) return rc;
+  }
   return DINT_OK;
 }
 

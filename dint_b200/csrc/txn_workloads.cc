@@ -1,514 +1,53 @@
-// txn_workloads.cc -- (part of libdint_wl.so) the reference's TATP and SmallBank closed-loop clients
-// restated as round-based generators: tatp/caladan/client_udp_shard.cc:177-1184 (seven transaction types,
-// mix 35/35/10/2/14/2/2, tatp/udp/tatp.h:57-63) and smallbank/caladan/client_udp_shard.cc:169-1300 (six
-// types, mix 15/15/15/25/15/15, hot-account skew smallbank/udp/smallbank.h:16-18,24-46).
+// txn_workloads.cc -- (part of libdint_wl.so) the HOST driver of the reference's TATP and SmallBank closed-loop clients
+// as round-based generators.  The state machines themselves are txn_clients.h, shared with the device driver
+// (txn_clients.cuh); see there for the transaction types, mixes and the reference code they restate.
 //
-// A ROUND = every logical client has the requests of its current protocol step outstanding (1-6 wire
-// records: the reference fans a step out to the shards in parallel and joins).  dint_txn_next() emits the
-// round -- each client's records contiguous, in the order the reference pushes them per shard -- plus the
-// destination shard of every record; dint_txn_feed() hands the replies back in the same layout and
-// advances every client's state machine.  Like the reference, each client draws from the LCG
-// fastrand(seed = 0xdeadbeef + client gid) (tatp/udp/tatp.h:32-42), so a client's transaction stream is
-// the reference's for that gid.
-//
-// Sharding generalised from 3 to G shards (SURVEY.md section 8(e)): primary p = key % G, backups
-// (p+1) % G and (p+2) % G, log records to those same three; G = 3 is exactly the reference.
+// A ROUND = every logical client has the requests of its current protocol step outstanding (1-9 wire
+// records).  dint_txn_next() emits the round -- each client's records contiguous, in the order the reference
+// pushes them per shard -- plus the destination shard of every record; dint_txn_feed() hands the replies back
+// in the same layout and advances every client's state machine.
 #include <cstdint>
 #include <cstring>
 #include <vector>
 
+#include "txn_clients.h"
+
+using namespace dint::txn;
+
 namespace {
 
-inline uint32_t fastrand(uint64_t* seed) {
-  *seed = *seed * 1103515245ULL + 12345ULL;
-  return (uint32_t)(*seed >> 32);
-}
-inline void put64(uint8_t* p, uint64_t v) { memcpy(p, &v, 8); }
-inline uint64_t get64(const uint8_t* p) { uint64_t v; memcpy(&v, p, 8); return v; }
-inline uint32_t get32(const uint8_t* p) { uint32_t v; memcpy(&v, p, 4); return v; }
-inline void put32(uint8_t* p, uint32_t v) { memcpy(p, &v, 4); }
-
-// ================================================ TATP ==============================================
-// wire: {ord@0, type@1, table@2, key@3, val@11[40], ver@51}  (tatp/udp/net.h:57-65)
-constexpr int TM = 55;
-enum { T_READ = 0, T_LOCK = 1, T_ABORT = 2, T_GRANT_READ = 4, T_NOT_EXIST = 6, T_GRANT_LOCK = 7, T_REJECT_LOCK = 8,
-       T_COMMIT_PRIM = 12, T_COMMIT_BCK = 13, T_COMMIT_LOG = 14, T_INSERT_PRIM = 18, T_INSERT_BCK = 19,
-       T_DELETE_PRIM = 22, T_DELETE_BCK = 23, T_DELETE_LOG = 24 };
-enum { TB_SUB = 0, TB_SEC = 1, TB_ACC = 2, TB_SF = 3, TB_CF = 4 };
-enum { X_GET_SUB = 0, X_GET_ACC, X_GET_DEST, X_UPD_SUB, X_UPD_LOC, X_INS_CF, X_DEL_CF };
-
-struct TMsg { uint8_t b[TM]; };
-
-inline uint64_t sub_nbr_of(uint32_t s_id) {            // tatp/udp/tatp.h:17-25,132-144
-  uint64_t r = 0;
-  for (int g = 0; g < 3; g++) {
-    uint32_t i = s_id % 1000;
-    s_id /= 1000;
-    r |= ((uint64_t)(((i / 100) % 10) << 8 | ((i / 10) % 10) << 4 | (i % 10))) << (12 * g);
+// the host sink: records appended to the round in push order, plus their destination shard
+struct Out {
+  uint8_t* req; uint8_t* dst; uint32_t n = 0; uint32_t msz = TM;
+  void push(const uint8_t* rec, uint32_t shard, int ord) {
+    memcpy(req + (size_t)n * msz, rec, msz);
+    if (ord >= 0) req[(size_t)n * msz] = (uint8_t)ord;       // msg->ord = j: index inside the shard's list
+    dst[n++] = (uint8_t)shard;
   }
-  return r;
-}
-
-struct TatpClient {
-  uint64_t seed;
-  uint8_t txn = 0, phase = 0, n_out = 0;
-  uint32_t s_id = 0, vlr = 0;
-  uint8_t sf_type = 0, start_time = 0, end_time = 0, cf_to_fetch = 0;
-  TMsg a, b, c, d;          // saved replies; roles depend on the transaction (see comments below)
-  bool lock_a = false, lock_b = false;
+};
+// the replies of one client: contiguous, in push order
+struct Contig {
+  const uint8_t* r; uint32_t msz;
+  const uint8_t* rec(int i) const { return r + (size_t)i * msz; }
 };
 
 }  // namespace
 
 struct dint_txn {
   int kind;                 // 4 = tatp, 5 = smallbank
-  uint32_t n_clients, G, subscribers, accounts, hot_accounts;
+  uint32_t n_clients;
+  Params P;
   std::vector<TatpClient> tc;
-  struct dint_sb* sb = nullptr;                          // smallbank clients
+  std::vector<SbClient> sc;
   uint64_t st_requests = 0, st_txns = 0, st_committed = 0, st_rounds = 0;
   uint64_t st_by_type[8] = {0}, st_commit_by_type[8] = {0};
 
-  uint32_t nurand(uint64_t* seed) const {               // tatp/udp/tatp.h:40-43
-    return ((fastrand(seed) % subscribers) | (fastrand(seed) & 1048575u)) % subscribers;
-  }
-
-  // ---- helpers ------------------------------------------------------------------------------------
-  static void mk(TMsg& m, uint8_t type, uint8_t table, uint64_t key) {
-    memset(m.b, 0, TM);
-    m.b[1] = type; m.b[2] = table; put64(m.b + 3, key);
-  }
-  struct Out {
-    uint8_t* req; uint8_t* dst; uint32_t n = 0; uint32_t per_shard[8] = {0}; uint32_t G; uint32_t msz = TM;
-    void push(const TMsg& m, uint32_t shard, bool set_ord) {
-      memcpy(req + (size_t)n * msz, m.b, msz);
-      if (set_ord) req[(size_t)n * msz] = (uint8_t)per_shard[shard % 8];    // msg->ord = j: index inside the shard's list
-      per_shard[shard % 8]++;
-      dst[n++] = (uint8_t)shard;
-    }
-  };
-  uint32_t prim(uint64_t key) const { return (uint32_t)(key % G); }
-
-  void begin_txn(TatpClient& c) {
-    static const uint8_t mix[100] = {
-#define R5(x) x, x, x, x, x
-#define R35(x) R5(x), R5(x), R5(x), R5(x), R5(x), R5(x), R5(x)
-        R35(X_GET_SUB), R35(X_GET_ACC), R5(X_GET_DEST), R5(X_GET_DEST), X_UPD_SUB, X_UPD_SUB,
-        R5(X_UPD_LOC), R5(X_UPD_LOC), X_UPD_LOC, X_UPD_LOC, X_UPD_LOC, X_UPD_LOC, X_INS_CF, X_INS_CF, X_DEL_CF, X_DEL_CF};
-#undef R35
-#undef R5
-    c.txn = mix[fastrand(&c.seed) % 100];               // client_udp_shard.cc:1144
-    c.phase = 0;
-    c.lock_a = c.lock_b = false;
-    st_txns++;
-    st_by_type[c.txn]++;
-    switch (c.txn) {                                     // transaction parameters, in the reference's draw order
-      case X_GET_SUB: c.s_id = nurand(&c.seed); break;
-      case X_GET_ACC: c.s_id = nurand(&c.seed); c.sf_type = (uint8_t)((fastrand(&c.seed) & 3) + 1); break;
-      case X_GET_DEST:
-      case X_INS_CF:
-        c.s_id = nurand(&c.seed);
-        c.sf_type = (uint8_t)((fastrand(&c.seed) % 4) + 1);
-        c.start_time = (uint8_t)((fastrand(&c.seed) % 3) * 8);
-        c.end_time = (uint8_t)(fastrand(&c.seed) % 24);
-        c.cf_to_fetch = (uint8_t)(c.start_time / 8 + 1);
-        break;
-      case X_UPD_SUB: c.s_id = nurand(&c.seed); c.sf_type = (uint8_t)((fastrand(&c.seed) % 4) + 1); break;
-      case X_UPD_LOC: c.s_id = nurand(&c.seed); c.vlr = fastrand(&c.seed); break;
-      default:  // X_DEL_CF
-        c.s_id = nurand(&c.seed);
-        c.sf_type = (uint8_t)((fastrand(&c.seed) % 4) + 1);
-        c.start_time = (uint8_t)((fastrand(&c.seed) % 3) * 8);
-        break;
-    }
-  }
-  void finish(TatpClient& c, bool committed) {
-    if (committed) { st_committed++; st_commit_by_type[c.txn]++; }
-    begin_txn(c);
-  }
-
-  uint64_t k_sub(const TatpClient& c) const { return c.s_id; }
-  uint64_t k_sf(const TatpClient& c) const { return (uint64_t)c.s_id | ((uint64_t)c.sf_type << 32); }
-  uint64_t k_cf(const TatpClient& c, uint32_t st) const { return k_sf(c) | ((uint64_t)st << 40); }
-
-  // Replication fan-out of up to two records.  Per-shard arrival order follows the reference's push order:
-  // log: for shard { rec0, rec1 } (:490-499); backups: rec0,rec1 -> +1 then rec0,rec1 -> +2 (:523-531).
-  void emit_log(Out& o, const TMsg* recs, int n, uint8_t type) {
-    for (uint32_t s = 0; s < G; s++)
-      for (int k = 0; k < n; k++) {
-        const uint32_t p = prim(get64(recs[k].b + 3));
-        for (uint32_t off = 0; off < 3; off++)
-          if ((p + off) % G == s) { TMsg t = recs[k]; t.b[1] = type; o.push(t, s, false); }
-      }
-  }
-  void emit_bck(Out& o, const TMsg* recs, int n, uint8_t type) {
-    for (uint32_t s = 0; s < G; s++)
-      for (uint32_t off = 1; off <= 2; off++)
-        for (int k = 0; k < n; k++)
-          if ((prim(get64(recs[k].b + 3)) + off) % G == s) { TMsg t = recs[k]; t.b[1] = type; o.push(t, s, false); }
-  }
-  void emit_prim(Out& o, const TMsg* recs, int n, uint8_t type) {
-    for (uint32_t s = 0; s < G; s++)
-      for (int k = 0; k < n; k++)
-        if (prim(get64(recs[k].b + 3)) == s) { TMsg t = recs[k]; t.b[1] = type; o.push(t, s, false); }
-  }
-
-  // ---- one protocol step of one client ------------------------------------------------------------
-  void tatp_emit(TatpClient& c, Out& o) {
-    const uint32_t n0 = o.n;
-    memset(o.per_shard, 0, sizeof o.per_shard);
-    TMsg m;
-    switch (c.txn) {
-      case X_GET_SUB: mk(m, T_READ, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), false); break;                 // :177-199
-      case X_GET_ACC: mk(m, T_READ, TB_ACC, k_sf(c)); o.push(m, prim(k_sf(c)), false); break;                   // :305-331 (ai_type in sf_type)
-      case X_GET_DEST:                                                                                            // :202-302
-        if (c.phase == 0) { mk(m, T_READ, TB_SF, k_sf(c)); o.push(m, prim(k_sf(c)), false); }
-        else for (uint32_t i = 0; i < c.cf_to_fetch; i++) { mk(m, T_READ, TB_CF, k_cf(c, i * 8)); o.push(m, prim(k_cf(c, i * 8)), true); }
-        break;
-      case X_UPD_SUB:                                                                                             // :334-571
-        switch (c.phase) {
-          case 0:   // a = sub read, b = sub lock, c = specfac read, d = specfac lock
-            mk(m, T_READ, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), true);
-            mk(m, T_LOCK, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), true);
-            mk(m, T_READ, TB_SF, k_sf(c)); o.push(m, prim(k_sf(c)), true);
-            mk(m, T_LOCK, TB_SF, k_sf(c)); o.push(m, prim(k_sf(c)), true);
-            break;
-          case 1: { TMsg t = c.b; t.b[1] = T_ABORT; o.push(t, prim(k_sub(c)), false); break; }                   // release sub lock
-          case 2: { TMsg t = c.d; t.b[1] = T_ABORT; o.push(t, prim(k_sf(c)), false); break; }                    // release specfac lock
-          case 3:   // verify
-            mk(m, T_READ, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), true);
-            mk(m, T_READ, TB_SF, k_sf(c)); o.push(m, prim(k_sf(c)), true);
-            break;
-          case 4: { TMsg rr[2] = {c.a, c.c}; emit_log(o, rr, 2, T_COMMIT_LOG); break; }      // :487-518
-          case 5: { TMsg rr[2] = {c.a, c.c}; emit_bck(o, rr, 2, T_COMMIT_BCK); break; }      // :520-548
-          default: { TMsg rr[2] = {c.a, c.c}; emit_prim(o, rr, 2, T_COMMIT_PRIM); break; }   // :550-568
-        }
-        break;
-      case X_UPD_LOC:                                                                                             // :574-728
-        switch (c.phase) {
-          case 0: mk(m, T_READ, TB_SEC, sub_nbr_of(c.s_id)); o.push(m, prim(sub_nbr_of(c.s_id)), false); break;
-          case 1:   // a = sub read, b = sub lock
-            mk(m, T_READ, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), true);
-            mk(m, T_LOCK, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), true);
-            break;
-          case 2: mk(m, T_READ, TB_SUB, k_sub(c)); o.push(m, prim(k_sub(c)), false); break;                      // verify
-          case 3: { TMsg t = c.b; t.b[1] = T_ABORT; o.push(t, prim(k_sub(c)), false); break; }
-          case 4: emit_log(o, &c.a, 1, T_COMMIT_LOG); break;
-          case 5: emit_bck(o, &c.a, 1, T_COMMIT_BCK); break;
-          default: emit_prim(o, &c.a, 1, T_COMMIT_PRIM); break;
-        }
-        break;
-      case X_INS_CF:                                                                                              // :731-951
-        switch (c.phase) {
-          case 0: mk(m, T_READ, TB_SEC, sub_nbr_of(c.s_id)); o.push(m, prim(sub_nbr_of(c.s_id)), false); break;
-          case 1: mk(m, T_READ, TB_SF, k_sf(c)); o.push(m, prim(k_sf(c)), false); break;                         // c = specfac read
-          case 2:   // a = callfwd read, b = callfwd lock
-            mk(m, T_READ, TB_CF, k_cf(c, c.start_time)); o.push(m, prim(k_cf(c, c.start_time)), true);
-            mk(m, T_LOCK, TB_CF, k_cf(c, c.start_time)); o.push(m, prim(k_cf(c, c.start_time)), true);
-            break;
-          case 3: { TMsg t = c.b; t.b[1] = T_ABORT; o.push(t, prim(k_cf(c, c.start_time)), false); break; }
-          case 4:   // verify specfac version + callfwd still absent
-            mk(m, T_READ, TB_SF, k_sf(c)); o.push(m, prim(k_sf(c)), true);
-            mk(m, T_READ, TB_CF, k_cf(c, c.start_time)); o.push(m, prim(k_cf(c, c.start_time)), true);
-            break;
-          case 5: emit_log(o, &c.a, 1, T_COMMIT_LOG); break;
-          case 6: emit_bck(o, &c.a, 1, T_INSERT_BCK); break;
-          default: emit_prim(o, &c.a, 1, T_INSERT_PRIM); break;
-        }
-        break;
-      default:  // X_DEL_CF                                                                                       // :954-1117
-        switch (c.phase) {
-          case 0: mk(m, T_READ, TB_SEC, sub_nbr_of(c.s_id)); o.push(m, prim(sub_nbr_of(c.s_id)), false); break;
-          case 1:   // a = callfwd read, b = callfwd lock
-            mk(m, T_READ, TB_CF, k_cf(c, c.start_time)); o.push(m, prim(k_cf(c, c.start_time)), true);
-            mk(m, T_LOCK, TB_CF, k_cf(c, c.start_time)); o.push(m, prim(k_cf(c, c.start_time)), true);
-            break;
-          case 2: { TMsg t = c.b; t.b[1] = T_ABORT; o.push(t, prim(k_cf(c, c.start_time)), false); break; }
-          case 3: mk(m, T_READ, TB_CF, k_cf(c, c.start_time)); o.push(m, prim(k_cf(c, c.start_time)), false); break;   // verify
-          case 4: emit_log(o, &c.a, 1, T_DELETE_LOG); break;
-          case 5: emit_bck(o, &c.a, 1, T_DELETE_BCK); break;
-          default: emit_prim(o, &c.a, 1, T_DELETE_PRIM); break;
-        }
-        break;
-    }
-    c.n_out = (uint8_t)(o.n - n0);
-  }
-
-  void tatp_absorb(TatpClient& c, const uint8_t* r) {
-    auto R = [&](int i) { TMsg m; memcpy(m.b, r + (size_t)i * TM, TM); return m; };
-    auto type = [&](int i) { return r[(size_t)i * TM + 1]; };
-    auto ver = [&](const TMsg& m) { return get32(m.b + 51); };
-    switch (c.txn) {
-      case X_GET_SUB: finish(c, true); break;
-      case X_GET_ACC: finish(c, type(0) == T_GRANT_READ); break;
-      case X_GET_DEST:
-        if (c.phase == 0) {
-          if (type(0) == T_NOT_EXIST || r[11] == 0) finish(c, false);      // record absent or is_active == 0 (:231-237)
-          else c.phase = 1;
-        } else {
-          bool ok = false;
-          for (uint32_t i = 0; i < c.cf_to_fetch; i++)
-            if (type(i) == T_GRANT_READ && i * 8 <= c.start_time && c.end_time < r[(size_t)i * TM + 11]) ok = true;   // :287-297
-          finish(c, ok);
-        }
-        break;
-      case X_UPD_SUB:
-        switch (c.phase) {
-          case 0:
-            c.a = R(0); c.b = R(1); c.c = R(2); c.d = R(3);
-            c.lock_a = type(1) == T_GRANT_LOCK; c.lock_b = type(3) == T_GRANT_LOCK;
-            if (type(2) == T_NOT_EXIST || !c.lock_a || !c.lock_b) {         // :400-420
-              if (c.lock_a) c.phase = 1; else if (c.lock_b) c.phase = 2; else finish(c, false);
-            } else {
-              uint16_t bits = (uint16_t)fastrand(&c.seed);                  // sub_val->bits (:425)
-              memcpy(c.a.b + 11 + 30, &bits, 2);
-              c.c.b[11 + 2] = (uint8_t)fastrand(&c.seed);                   // specfac_val->data_a (:429)
-              c.phase = 3;
-            }
-            break;
-          case 1: if (c.lock_b) c.phase = 2; else finish(c, false); break;
-          case 2: finish(c, false); break;
-          case 3:
-            if (ver(c.a) != get32(r + 51) || ver(c.c) != get32(r + TM + 51)) { c.phase = 1; }   // abort both (:470-484)
-            else {
-              put32(c.a.b + 51, ver(c.a) + 1); put32(c.c.b + 51, ver(c.c) + 1);                   // :487-488
-              c.phase = 4;
-            }
-            break;
-          case 4: c.phase = 5; break;
-          case 5: c.phase = 6; break;
-          default: finish(c, true); break;
-        }
-        break;
-      case X_UPD_LOC:
-        switch (c.phase) {
-          case 0: c.phase = 1; break;
-          case 1:
-            c.a = R(0); c.b = R(1);
-            if (type(1) == T_REJECT_LOCK) finish(c, false);                  // :642
-            else { memcpy(c.a.b + 11 + 36, &c.vlr, 4); c.phase = 2; }        // sub_val->vlr_location (:646)
-            break;
-          case 2:
-            if (get32(r + 51) != ver(c.a)) c.phase = 3;                      // :661-667
-            else { put32(c.a.b + 51, ver(c.a) + 1); c.phase = 4; }
-            break;
-          case 3: finish(c, false); break;
-          case 4: c.phase = 5; break;
-          case 5: c.phase = 6; break;
-          default: finish(c, true); break;
-        }
-        break;
-      case X_INS_CF:
-        switch (c.phase) {
-          case 0: c.phase = 1; break;
-          case 1: c.c = R(0); if (type(0) == T_NOT_EXIST) finish(c, false); else c.phase = 2; break;   // :781
-          case 2:
-            c.a = R(0); c.b = R(1);
-            if (type(0) == T_GRANT_READ || type(1) == T_REJECT_LOCK) {       // :831-841: row exists or lock refused
-              if (type(1) == T_GRANT_LOCK) c.phase = 3; else finish(c, false);
-            } else {
-              c.a.b[11 + 1] = 101;                                           // numberx[0] = magic (:846)
-              c.a.b[11 + 0] = c.end_time;                                    // end_time (:847)
-              c.phase = 4;
-            }
-            break;
-          case 3: finish(c, false); break;
-          case 4:
-            if (ver(c.c) != get32(r + 51) || type(1) == T_GRANT_READ) c.phase = 3;   // :884-891
-            else { put32(c.a.b + 51, 0); c.phase = 5; }                      // :894 ver = 0
-            break;
-          case 5: c.phase = 6; break;
-          case 6: c.phase = 7; break;
-          default: finish(c, true); break;
-        }
-        break;
-      default:  // X_DEL_CF
-        switch (c.phase) {
-          case 0: c.phase = 1; break;
-          case 1:
-            c.a = R(0); c.b = R(1);
-            if (type(0) == T_NOT_EXIST || type(1) == T_REJECT_LOCK) {        // :1024-1033
-              if (type(1) == T_GRANT_LOCK) c.phase = 2; else finish(c, false);
-            } else c.phase = 3;
-            break;
-          case 2: finish(c, false); break;
-          case 3:
-            if (type(0) == T_NOT_EXIST || get32(r + 51) != ver(c.a)) c.phase = 2;   // :1053-1060
-            else c.phase = 4;
-            break;
-          case 4: c.phase = 5; break;
-          case 5: c.phase = 6; break;
-          default: finish(c, true); break;
-        }
-        break;
-    }
-  }
-};
-
-// ================================================ SmallBank =========================================
-// wire: {ord@0, type@1, table@2, key@3, val@11[8] = {u32 magic; float bal}, ver@19}  (smallbank/udp/net.h:43-52)
-namespace {
-constexpr int SMSZ = 23;
-enum { S_ACQ_S = 0, S_ACQ_X = 1, S_REL_S = 2, S_REL_X = 3, S_COMMIT_PRIM = 4, S_COMMIT_BCK = 5, S_COMMIT_LOG = 6,
-       S_GRANT_S = 7, S_REJECT_S = 8, S_GRANT_X = 9, S_REJECT_X = 10 };
-enum { B_AMALGAMATE = 0, B_BALANCE, B_DEPOSIT, B_SEND, B_TRANSACT, B_WRITECHECK };
-enum { SP_ACQ = 0, SP_REL_ABORT, SP_LOG, SP_BCK, SP_PRIM, SP_RELEASE };
-struct SbRow { uint8_t table, excl, write, granted; uint64_t acct; TMsg m; };
-struct SbClient {
-  uint64_t seed;
-  uint8_t txn = 0, phase = 0, n_rows = 0, n_out = 0, rel_idx = 0;
-  SbRow r[3];
-};
-inline float get_bal(const TMsg& m) { float f; memcpy(&f, m.b + 11 + 4, 4); return f; }
-inline void set_bal(TMsg& m, float f) { memcpy(m.b + 11 + 4, &f, 4); }
-}  // namespace
-
-struct dint_sb {
-  dint_txn* base;
-  std::vector<SbClient> cl;
-  uint32_t accounts, hot_accounts, G;
-
-  void get_account(uint64_t* seed, uint64_t* a) const {                 // smallbank/udp/smallbank.h:24-30
-    if (fastrand(seed) % 100 < 90) *a = fastrand(seed) % hot_accounts; else *a = fastrand(seed) % accounts;
-  }
-  void get_two_accounts(uint64_t* seed, uint64_t* a0, uint64_t* a1) const {   // smallbank.h:32-46
-    const uint32_t n = (fastrand(seed) % 100 < 90) ? hot_accounts : accounts;
-    *a0 = fastrand(seed) % n;
-    *a1 = fastrand(seed) % n;
-    while (*a1 == *a0) *a1 = fastrand(seed) % n;
-  }
-  static void row(SbRow& r, uint8_t table, bool excl, bool write, uint64_t acct) {
-    r.table = table; r.excl = excl; r.write = write; r.granted = 0; r.acct = acct;
-  }
-  void begin(SbClient& c) {
-    static const uint8_t mix[100] = {
-#define R5(x) x, x, x, x, x
-#define R15(x) R5(x), R5(x), R5(x)
-        R15(B_AMALGAMATE), R15(B_BALANCE), R15(B_DEPOSIT), R15(B_SEND), R5(B_SEND), R5(B_SEND), R15(B_TRANSACT), R15(B_WRITECHECK)};
-#undef R15
-#undef R5
-    c.txn = mix[fastrand(&c.seed) % 100];
-    c.phase = SP_ACQ;
-    base->st_txns++;
-    base->st_by_type[c.txn]++;
-    uint64_t a0, a1;
-    switch (c.txn) {
-      case B_AMALGAMATE:       // client_udp_shard.cc:169-438: sav(a0) X, chk(a0) X, chk(a1) X, all written
-        get_two_accounts(&c.seed, &a0, &a1);
-        c.n_rows = 3; row(c.r[0], 0, true, true, a0); row(c.r[1], 1, true, true, a0); row(c.r[2], 1, true, true, a1);
-        break;
-      case B_BALANCE:          // :441-578: sav(a) S, chk(a) S, read only
-        get_account(&c.seed, &a0);
-        c.n_rows = 2; row(c.r[0], 0, false, false, a0); row(c.r[1], 1, false, false, a0);
-        break;
-      case B_DEPOSIT:          // :581-684: chk(a) X += 1.3
-        get_account(&c.seed, &a0);
-        c.n_rows = 1; row(c.r[0], 1, true, true, a0);
-        break;
-      case B_SEND:             // :687-932: chk(a0) X, chk(a1) X, move 5.0
-        get_two_accounts(&c.seed, &a0, &a1);
-        c.n_rows = 2; row(c.r[0], 1, true, true, a0); row(c.r[1], 1, true, true, a1);
-        break;
-      case B_TRANSACT:         // :935-1038: sav(a) X += 20.20
-        get_account(&c.seed, &a0);
-        c.n_rows = 1; row(c.r[0], 0, true, true, a0);
-        break;
-      default:                 // B_WRITECHECK :1041-1239: sav(a) S, chk(a) X -= 5 (+1 penalty)
-        get_account(&c.seed, &a0);
-        c.n_rows = 2; row(c.r[0], 0, false, false, a0); row(c.r[1], 1, true, true, a0);
-        break;
-    }
-  }
-  void finish(SbClient& c, bool ok) {
-    if (ok) { base->st_committed++; base->st_commit_by_type[c.txn]++; }
-    begin(c);
-  }
-  void emit(SbClient& c, dint_txn::Out& o) {
-    const uint32_t n0 = o.n;
-    memset(o.per_shard, 0, sizeof o.per_shard);
-    TMsg rr[3];
-    int nw = 0;
-    for (int i = 0; i < c.n_rows; i++) if (c.r[i].write) rr[nw++] = c.r[i].m;
-    switch (c.phase) {
-      case SP_ACQ:
-        for (int i = 0; i < c.n_rows; i++) {
-          TMsg m; memset(m.b, 0, sizeof m.b);
-          m.b[1] = c.r[i].excl ? S_ACQ_X : S_ACQ_S; m.b[2] = c.r[i].table; put64(m.b + 3, c.r[i].acct);
-          o.push(m, (uint32_t)(c.r[i].acct % G), c.n_rows > 1);
-        }
-        break;
-      case SP_REL_ABORT: {
-        TMsg m = c.r[c.rel_idx].m; m.b[1] = c.r[c.rel_idx].excl ? S_REL_X : S_REL_S;
-        o.push(m, (uint32_t)(c.r[c.rel_idx].acct % G), false);
-        break;
-      }
-      case SP_LOG: base->emit_log(o, rr, nw, S_COMMIT_LOG); break;
-      case SP_BCK: base->emit_bck(o, rr, nw, S_COMMIT_BCK); break;
-      case SP_PRIM: base->emit_prim(o, rr, nw, S_COMMIT_PRIM); break;
-      default:
-        for (int i = 0; i < c.n_rows; i++) {
-          TMsg m = c.r[i].m; m.b[1] = c.r[i].excl ? S_REL_X : S_REL_S;
-          o.push(m, (uint32_t)(c.r[i].acct % G), c.n_rows > 1);
-        }
-        break;
-    }
-    c.n_out = (uint8_t)(o.n - n0);
-  }
-  int next_granted(const SbClient& c, int from) const {
-    for (int i = from; i < c.n_rows; i++) if (c.r[i].granted) return i;
-    return -1;
-  }
-  void absorb(SbClient& c, const uint8_t* r) {
-    switch (c.phase) {
-      case SP_ACQ: {
-        bool all = true;
-        for (int i = 0; i < c.n_rows; i++) {
-          memcpy(c.r[i].m.b, r + (size_t)i * SMSZ, SMSZ);
-          const uint8_t t = c.r[i].m.b[1];
-          c.r[i].granted = (t == S_GRANT_S || t == S_GRANT_X);
-          all &= (bool)c.r[i].granted;
-        }
-        bool logic_abort = false;
-        if (all) {
-          TMsg& m0 = c.r[0].m;
-          switch (c.txn) {
-            case B_AMALGAMATE:
-              set_bal(c.r[2].m, get_bal(c.r[2].m) + (get_bal(c.r[0].m) + get_bal(c.r[1].m)));
-              set_bal(c.r[0].m, 0.f); set_bal(c.r[1].m, 0.f);
-              break;
-            case B_DEPOSIT: set_bal(m0, get_bal(m0) + 1.3f); break;
-            case B_SEND:
-              if (get_bal(c.r[0].m) < 5.0f) logic_abort = true;
-              else { set_bal(c.r[0].m, get_bal(c.r[0].m) - 5.0f); set_bal(c.r[1].m, get_bal(c.r[1].m) + 5.0f); }
-              break;
-            case B_TRANSACT: set_bal(m0, get_bal(m0) + 20.20f); break;
-            case B_WRITECHECK:
-              if (get_bal(c.r[0].m) + get_bal(c.r[1].m) < 5.0f) set_bal(c.r[1].m, get_bal(c.r[1].m) - 6.0f);
-              else set_bal(c.r[1].m, get_bal(c.r[1].m) - 5.0f);
-              break;
-            default: break;
-          }
-        }
-        if (!all || logic_abort) {
-          int g = next_granted(c, 0);
-          if (g < 0) finish(c, false); else { c.rel_idx = (uint8_t)g; c.phase = SP_REL_ABORT; }
-        } else if (c.txn == B_BALANCE) {
-          c.phase = SP_RELEASE;
-        } else {
-          for (int i = 0; i < c.n_rows; i++) if (c.r[i].write) put32(c.r[i].m.b + 19, get32(c.r[i].m.b + 19) + 1);   // ver++
-          c.phase = SP_LOG;
-        }
-        break;
-      }
-      case SP_REL_ABORT: {
-        int g = next_granted(c, c.rel_idx + 1);
-        if (g < 0) finish(c, false); else c.rel_idx = (uint8_t)g;
-        break;
-      }
-      case SP_LOG: c.phase = SP_BCK; break;
-      case SP_BCK: c.phase = SP_PRIM; break;
-      case SP_PRIM: c.phase = SP_RELEASE; break;
-      default: finish(c, true); break;
-    }
+  void began(uint8_t txn) { st_txns++; st_by_type[txn]++; }
+  // ev: what absorb returned; new_txn: the client's transaction after it
+  void count(int ev, uint8_t new_txn) {
+    if (ev < 0) return;
+    if (ev & 1) { st_committed++; st_commit_by_type[ev >> 1]++; }
+    began(new_txn);
   }
 };
 
@@ -521,47 +60,54 @@ dint_txn* dint_txn_create(int kind, uint32_t n_clients, uint32_t gid0, uint32_t 
   // primary + 2 distinct backups need >= 3 shards; 1 = everything on one server (three copies of each write)
   if ((kind != 4 && kind != 5) || n_clients == 0 || n_shards == 0 || n_shards == 2 || n_shards > 8 || subscribers < 3) return nullptr;
   dint_txn* w = new dint_txn();
-  w->kind = kind; w->n_clients = n_clients; w->G = n_shards; w->subscribers = subscribers;
+  w->kind = kind; w->n_clients = n_clients;
+  w->P.G = n_shards; w->P.subscribers = subscribers; w->P.accounts = subscribers; w->P.hot = sb_hot_accounts(subscribers);
   if (kind == 4) {
-    w->tc.resize(n_clients);
+    w->tc.assign(n_clients, TatpClient{});
     for (uint32_t i = 0; i < n_clients; i++) {
       w->tc[i].seed = 0xdeadbeefULL + gid0 + i;              // client_udp_shard.cc:1121
-      w->begin_txn(w->tc[i]);
+      tatp_begin(w->P, w->tc[i]);
+      w->began(w->tc[i].txn);
     }
   } else {
-    dint_sb* sb = new dint_sb();
-    sb->base = w; sb->G = n_shards; sb->accounts = subscribers;
-    sb->hot_accounts = (uint32_t)((uint64_t)subscribers * 960000 / 24000000);   // kHotAccountNum / kAccountNum
-    if (sb->hot_accounts < 2) sb->hot_accounts = 2;
-    sb->cl.resize(n_clients);
-    for (uint32_t i = 0; i < n_clients; i++) { sb->cl[i].seed = 0xdeadbeefULL + gid0 + i; sb->begin(sb->cl[i]); }
-    w->sb = sb;
+    w->sc.assign(n_clients, SbClient{});
+    for (uint32_t i = 0; i < n_clients; i++) {
+      w->sc[i].seed = 0xdeadbeefULL + gid0 + i;
+      sb_begin(w->P, w->sc[i]);
+      w->began(w->sc[i].txn);
+    }
   }
   return w;
 }
-void dint_txn_destroy(dint_txn* w) { if (w) delete w->sb; delete w; }
+void dint_txn_destroy(dint_txn* w) { delete w; }
 uint32_t dint_txn_max_round(const dint_txn* w) { return w->n_clients * 9; }
 
 // emits one round; returns the number of wire records.  req: capacity dint_txn_max_round() records;
 // dst[i] = destination shard of record i.
 uint64_t dint_txn_next(dint_txn* w, void* req, uint8_t* dst) {
-  dint_txn::Out o;
-  o.req = (uint8_t*)req; o.dst = dst; o.G = w->G;
-  if (w->sb) { o.msz = SMSZ; for (auto& c : w->sb->cl) w->sb->emit(c, o); }
-  else for (auto& c : w->tc) w->tatp_emit(c, o);
+  Out o;
+  o.req = (uint8_t*)req; o.dst = dst;
+  if (w->kind == 5) { o.msz = SMSZ; for (auto& c : w->sc) c.n_out = (uint8_t)sb_emit(w->P, c, o); }
+  else for (auto& c : w->tc) c.n_out = (uint8_t)tatp_emit(w->P, c, o);
   w->st_requests += o.n;
   w->st_rounds++;
   return o.n;
 }
 void dint_txn_feed(dint_txn* w, const void* resp) {
   const uint8_t* r = (const uint8_t*)resp;
-  if (w->sb) {
-    for (auto& c : w->sb->cl) { const uint32_t n = c.n_out; w->sb->absorb(c, r); r += (size_t)n * SMSZ; }
+  if (w->kind == 5) {
+    for (auto& c : w->sc) {
+      const uint32_t n = c.n_out;        // read before absorb: it may start a new transaction
+      const int ev = sb_absorb(w->P, c, Contig{r, SMSZ});
+      w->count(ev, c.txn);                 // c.txn is read after absorb: the transaction it began
+      r += (size_t)n * SMSZ;
+    }
     return;
   }
   for (auto& c : w->tc) {
-    const uint32_t n = c.n_out;          // absorb may start a new transaction and must not see its own n_out
-    w->tatp_absorb(c, r);
+    const uint32_t n = c.n_out;
+    const int ev = tatp_absorb(w->P, c, Contig{r, TM});
+    w->count(ev, c.txn);
     r += (size_t)n * TM;
   }
 }

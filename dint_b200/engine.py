@@ -50,7 +50,7 @@ _lib = None
 # every symbol include/dint_b200.h declares
 ABI_SYMBOLS = [
     "dint_msg_size", "dint_default_cfg", "dint_create", "dint_destroy", "dint_populate", "dint_load",
-    "dint_submit", "dint_submit_device", "dint_route_owner", "dint_route_partition", "dint_route_unpermute", "dint_route_tile_records", "dint_route_dispatch", "dint_route_combine", "dint_p2p_wait", "dint_p2p_signal", "dint_shard_create", "dint_shard_destroy", "dint_shard_submit_many", "dint_shard_submit_host", "dint_shard_submit_many_v", "dint_shard_flags", "dint_cluster_create", "dint_cluster_populate", "dint_cluster_submit", "dint_cluster_engine", "dint_cluster_size", "dint_cluster_overflow_retries", "dint_shard_recover", "dint_cluster_destroy", "dint_clients_create", "dint_clients_run", "dint_clients_stats", "dint_clients_peek", "dint_clients_destroy", "dint_snapshot_create", "dint_snapshot_restore", "dint_snapshot_destroy", "dint_sync", "dint_kv_get", "dint_kv_count", "dint_lock_state",
+    "dint_submit", "dint_submit_device", "dint_route_owner", "dint_route_partition", "dint_route_unpermute", "dint_route_tile_records", "dint_route_dispatch", "dint_route_combine", "dint_p2p_wait", "dint_p2p_signal", "dint_shard_create", "dint_shard_destroy", "dint_shard_submit_many", "dint_shard_submit_host", "dint_shard_submit_many_v", "dint_shard_flags", "dint_cluster_create", "dint_cluster_populate", "dint_cluster_submit", "dint_cluster_engine", "dint_cluster_size", "dint_cluster_overflow_retries", "dint_shard_recover", "dint_cluster_destroy", "dint_clients_create", "dint_clients_run", "dint_clients_stats", "dint_clients_peek", "dint_clients_destroy", "dint_txn_clients_create", "dint_txn_clients_run", "dint_txn_clients_stats", "dint_txn_clients_peek", "dint_txn_clients_destroy", "dint_snapshot_create", "dint_snapshot_restore", "dint_snapshot_destroy", "dint_sync", "dint_kv_get", "dint_kv_count", "dint_lock_state",
     "dint_lock_slot", "dint_dump_log", "dint_log_entry_size", "dint_get_stats", "dint_reset_stats",
     "dint_profile", "dint_kernel_times", "dint_last_error", "dint_host_alloc", "dint_host_free",
     "dint_test_fasthash64", "dint_test_fastmod", "dint_test_host_slices",
@@ -101,6 +101,11 @@ def lib():
     L.dint_clients_stats.restype = i32; L.dint_clients_stats.argtypes = [vp, C.POINTER(u64)]
     L.dint_clients_peek.restype = i32; L.dint_clients_peek.argtypes = [vp, vp, vp]
     L.dint_clients_destroy.restype = None; L.dint_clients_destroy.argtypes = [vp]
+    L.dint_txn_clients_create.restype = i32; L.dint_txn_clients_create.argtypes = [C.POINTER(vp), u32, u32, u32, u32, C.POINTER(vp)]
+    L.dint_txn_clients_run.restype = i32; L.dint_txn_clients_run.argtypes = [vp, u32, vp]
+    L.dint_txn_clients_stats.restype = i32; L.dint_txn_clients_stats.argtypes = [vp, C.POINTER(u64)]
+    L.dint_txn_clients_peek.restype = i32; L.dint_txn_clients_peek.argtypes = [vp, vp, vp, vp, C.POINTER(u64)]
+    L.dint_txn_clients_destroy.restype = None; L.dint_txn_clients_destroy.argtypes = [vp]
     L.dint_snapshot_create.restype = i32; L.dint_snapshot_create.argtypes = [vp, C.POINTER(vp)]
     L.dint_snapshot_restore.restype = i32; L.dint_snapshot_restore.argtypes = [vp, vp]
     L.dint_snapshot_destroy.restype = None; L.dint_snapshot_destroy.argtypes = [vp]
@@ -449,6 +454,76 @@ class GpuClients:
         if getattr(self, "h", None):
             lib().dint_clients_destroy(self.h)
             self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class GpuTxnClients:
+    """TATP / SmallBank closed-loop clients resident on the GPU, driving the shard engines `engines` (engine i = shard i,
+    all of one kind, on one device) -- dint_txn_clients_*.  Same clients, draw for draw, as
+    dint_b200.txn_workloads.TxnWorkload(kind, n_clients, len(engines), subscribers, gid0)."""
+
+    def __init__(self, engines, n_clients, subscribers=None, gid0=0):
+        from .wire import TATP
+        self.engines = list(engines)
+        self.kind, self.msg = self.engines[0].kind, self.engines[0].msg
+        if subscribers is None:
+            subscribers = 7_000_000 if self.kind == TATP else 24_000_000
+        arr = (C.c_void_p * len(self.engines))(*[e.h.value for e in self.engines])
+        h = C.c_void_p()
+        rc = lib().dint_txn_clients_create(arr, len(self.engines), n_clients, gid0, subscribers, C.byref(h))
+        if rc != 0:
+            raise DintError(rc, "dint_txn_clients_create")
+        self.h = h
+
+    def run(self, rounds, stream=None):
+        """`rounds` closed-loop rounds on `stream` (default: the current torch stream); returns when the last round's
+        requests are written (one host sync per round)."""
+        if stream is None:
+            import torch
+            stream = torch.cuda.current_stream().cuda_stream
+        rc = lib().dint_txn_clients_run(self.h, rounds, C.c_void_p(stream) if stream else None)
+        if rc != 0:
+            raise DintError(rc, "dint_txn_clients_run")
+
+    def stats(self):
+        """The dict TxnWorkload.stats() returns: requests, txns, committed, rounds, by_type {name: (begun, committed)}."""
+        from .txn_workloads import stats_dict
+        out = (C.c_uint64 * 18)()
+        rc = lib().dint_txn_clients_stats(self.h, out)
+        if rc != 0:
+            raise DintError(rc, "dint_txn_clients_stats")
+        return stats_dict(self.kind, out)
+
+    def peek(self):
+        """(requests uint8 [n * msg], destination shard uint8 [n], last round's replies uint8 [m * msg]) in client order:
+        what TxnWorkload.next() returns for the pending round, and what was fed for the last one."""
+        n = (C.c_uint64 * 2)()
+        rc = lib().dint_txn_clients_peek(self.h, None, None, None, n)
+        if rc != 0:
+            raise DintError(rc, "dint_txn_clients_peek")
+        rq = np.empty(max(int(n[0]), 1) * self.msg, dtype=np.uint8)
+        dst = np.empty(max(int(n[0]), 1), dtype=np.uint8)
+        rs = np.empty(max(int(n[1]), 1) * self.msg, dtype=np.uint8)
+        rc = lib().dint_txn_clients_peek(self.h, rq.ctypes.data, dst.ctypes.data, rs.ctypes.data, n)
+        if rc != 0:
+            raise DintError(rc, "dint_txn_clients_peek")
+        return rq[: int(n[0]) * self.msg], dst[: int(n[0])], rs[: int(n[1]) * self.msg]
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().dint_txn_clients_destroy(self.h)
+            self.h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
 
     def __del__(self):
         try:

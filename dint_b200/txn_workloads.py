@@ -77,10 +77,15 @@ class TxnWorkload:
     def stats(self):
         out = (C.c_uint64 * 18)()
         lib().dint_txn_stats(self.h, out)
-        d = {"requests": int(out[0]), "txns": int(out[1]), "committed": int(out[2]), "rounds": int(out[3])}
-        names = TATP_TXN_NAMES if self.kind == TATP else SMALLBANK_TXN_NAMES
-        d["by_type"] = {n: (int(out[4 + i]), int(out[11 + i])) for i, n in enumerate(names)}
-        return d
+        return stats_dict(self.kind, out)
+
+
+def stats_dict(kind, out):
+    """The dint_txn_stats layout (18 counters) as a dict; by_type[name] = (begun, committed)."""
+    d = {"requests": int(out[0]), "txns": int(out[1]), "committed": int(out[2]), "rounds": int(out[3])}
+    names = TATP_TXN_NAMES if kind == TATP else SMALLBANK_TXN_NAMES
+    d["by_type"] = {n: (int(out[4 + i]), int(out[11 + i])) for i, n in enumerate(names)}
+    return d
 
 
 def partition_by_shard(req, dst, n_shards, msg):

@@ -285,6 +285,39 @@ int dint_clients_stats(dint_clients *c, uint64_t out[5]);
 int dint_clients_peek(dint_clients *c, void *next_req_host, void *last_resp_host);
 void dint_clients_destroy(dint_clients *c);
 
+/*
+ * TATP and SmallBank closed-loop clients ON the GPU (SURVEY.md section 8(f) rank 2).  The reference's clients are Caladan
+ * uthreads on other machines (tatp/caladan/client_udp_shard.cc:177-1184, smallbank/caladan/client_udp_shard.cc:169-1300):
+ * each runs one transaction at a time, fanning every protocol step out to the shard servers -- primary key % G, backups
+ * +1 and +2, the commit log on all three -- and joining on the replies.  Here n_clients of those state machines live on
+ * the device of the shard engines, one thread each, and drive them round after round, so committed txn/s and the abort
+ * rate per transaction type come from a live closed loop.  The state machines are the host clients' own
+ * (dint_b200/csrc/txn_clients.h, shared with dint_txn_* of libdint_wl.so): same gids (gid0 + i), same fastrand streams,
+ * the same requests in the same order, shard by shard.
+ *   dint_txn_clients_create: shards[i] = engine of shard i, all tatp or all smallbank, all on one device; n_shards = 1 or
+ *     3..8 (primary + 2 distinct backups); with n_shards > 3, engine i must be configured with txn_shards = n_shards and
+ *     txn_shard_id = i.  subscribers: kSubscriberNum (tatp, reference 7,000,000) or kAccountNum (smallbank, 24,000,000)
+ *     of the key generators -- what the engines populated.  n_clients <= 2^26.  Every client begins its first
+ *     transaction and emits its first round (synchronises).
+ *   dint_txn_clients_run: `rounds` rounds on cuda_stream.  A round = each shard engine serves the records pending for it
+ *     (dint_submit_device; empty shards are skipped), then three client kernels absorb the replies and write the next
+ *     round's records into the per-shard buffers.  The host reads the per-shard record counts once per round (the
+ *     engines size their launches on the host), so the call returns when the last round's records are written.
+ *   dint_txn_clients_stats (synchronises): the dint_txn_stats layout -- requests served, transactions begun, committed,
+ *     rounds served, begun by type[7], committed by type[7].
+ *   dint_txn_clients_peek (test hook, synchronises): the pending round's requests and destination shards, and the last
+ *     round's replies, in client order (each client's records contiguous, in push order), as dint_txn_next / dint_txn_feed
+ *     lay them out.  n_out = {pending records, replies of the last round}; NULL buffers: sizes only.
+ */
+typedef struct dint_txn_clients dint_txn_clients;
+int dint_txn_clients_create(dint_engine *const *shards, uint32_t n_shards, uint32_t n_clients, uint32_t gid0,
+                            uint32_t subscribers, dint_txn_clients **out);
+int dint_txn_clients_run(dint_txn_clients *c, uint32_t rounds, void *cuda_stream);
+int dint_txn_clients_stats(dint_txn_clients *c, uint64_t out[18]);
+int dint_txn_clients_peek(dint_txn_clients *c, void *next_req_host, uint8_t *next_dst_host, void *last_resp_host,
+                          uint64_t n_out[2]);
+void dint_txn_clients_destroy(dint_txn_clients *c);
+
 int dint_get_stats(dint_engine *e, dint_stats *s);
 void dint_reset_stats(dint_engine *e);
 /* per-kernel CUDA-event timing: 0 = off, 1 = every kernel, otherwise a bit mask over
